@@ -40,6 +40,7 @@ H, W, K_NEIGH = HP // 4, WP // 4, 8
 N_INST = B_IMG * GTS * INST_PER_GT
 ALGO_BYTES = 3 * N_INST * H * W * 4 + 2 * B_IMG * K_NEIGH * H * W * 4     # SURVEY section 8d: 85.2 MB / step
 ROTATE = 8
+DUMP_BYTES = 64 * 10 ** 6      # --dump-outputs: the most it writes
 
 
 def ncu_traffic_bytes():
@@ -158,6 +159,23 @@ def ddp_allreduce_leg(dist, dev, world, loss_step, steps):
             'exposed_comm_us': max(ms_both - ms_loss, 0.0) * 1e3,
             'what': 'fp32 gradient all-reduce of BoxInst R-50 (136 MB, 25 MB buckets, NCCL, async) overlapped with the eager '
                     'mask-loss step; reported next to the replica metric, not folded into it (the loss itself has no collective)'}
+
+
+def dump_outputs(out_dir, arrays):
+    """Writes what the timed path returned in its last step as <out_dir>/<name>.npy (float64 stays float64, every other dtype
+    becomes float32), so that two builds can be compared output for output on the same seeded inputs.  When the arrays exceed
+    DUMP_BYTES together, each one larger than an equal share of it is replaced by the same seeded sample of its flattened
+    elements on every run."""
+    import numpy as np
+    os.makedirs(out_dir, exist_ok=True)
+    arrays = {k: v.detach().cpu().numpy().astype(np.float64 if v.dtype == torch.float64 else np.float32)
+              for k, v in arrays.items()}
+    share = DUMP_BYTES // len(arrays) - 4096          # room for the .npy header
+    over = sum(a.nbytes for a in arrays.values()) > DUMP_BYTES - 4096 * len(arrays)
+    for name, a in arrays.items():
+        if over and a.nbytes > share:
+            a = a.reshape(-1)[np.sort(np.random.default_rng(0).choice(a.size, share // a.itemsize, replace=False))]
+        np.save(os.path.join(out_dir, name + '.npy'), a)
 
 
 def reduce_max_over_ranks(values, dist, device):
@@ -336,13 +354,13 @@ def main_cuda(args, rank, world, local_rank):
                                              for _ in range(ROTATE - 1)]
     logit_sets = [t.requires_grad_(True) for t in logit_sets]
     ones = torch.ones((), device=dev)
-    grad_ring = [None] * ROTATE       # keeps the last R gradients alive so every step writes a fresh 26 MB
+    out_ring = [None] * ROTATE        # keeps the last R outputs alive so every step writes a fresh 26 MB gradient
 
     def step(i):
         x = logit_sets[i % ROTATE]
         prj, pair = boxinst_mask_loss(x, targets, gt_inds32, it, plan=plan)
         torch.autograd.backward([prj, pair], [ones, ones])
-        grad_ring[i % ROTATE], x.grad = x.grad, None
+        out_ring[i % ROTATE], x.grad = (prj.detach(), pair.detach(), x.grad), None
         return prj, pair
 
     def barrier():
@@ -364,6 +382,7 @@ def main_cuda(args, rank, world, local_rank):
     for i in range(warm):
         step(i)
     ms_eager = timed(step, args.steps)
+    last = out_ring[(args.steps - 1) % ROTATE]      # (loss_prj, loss_pairwise, d/d mask logits) of the last timed step
 
     # ---- the same step (public autograd op, forward + backward) captured once per rotating input set
     #      into CUDA graphs: removes the ~0.2 ms/step of Python/autograd launch overhead ----
@@ -408,6 +427,7 @@ def main_cuda(args, rank, world, local_rank):
         REGIONS = 15
         samples = sorted(timed(region, 1) for _ in range(REGIONS))
         ms_step = samples[REGIONS // 2] / args.steps
+        last = graphs[-1]                       # the last step of the last graph a region replays
         ms_step_spread = (samples[0] / args.steps, samples[-1] / args.steps)
         steps_timed = args.steps
         mode = f'cuda_graph ({ROTATE} steps per graph' + (f' + one tail graph of {tail}' if tail else '') + \
@@ -531,6 +551,8 @@ def main_cuda(args, rank, world, local_rank):
         if dist is not None:
             dist.destroy_process_group()
         return
+    if args.dump_outputs:
+        dump_outputs(args.dump_outputs, dict(zip(('loss_prj', 'loss_pairwise', 'grad_mask_logits'), last)))
 
     peak, peak_src = measured_peak_gbs()
     achieved = ALGO_BYTES / (ms_step * 1e-3) / 1e9
@@ -662,10 +684,19 @@ def main_config(args, rank, world, local_rank):
     warm = max(args.warmup, 3)
     for i in range(max(warm, R)):
         steps_fn[i % R]()
-    steps = max(args.steps, 1)
-    ms_eager = timed(lambda i: steps_fn[i % R](), steps)
+    steps = args.steps
+    eager_last = []
+
+    def eager_step(i):
+        out = steps_fn[i % R]()
+        if i == steps - 1:                        # kept without its autograd graph, which would break the capture below
+            losses, grads = out
+            eager_last.append(({k: v.detach() for k, v in losses.items()} if isinstance(losses, dict) else losses.detach(),
+                               grads))
+    ms_eager = timed(eager_step, steps)
+    last = eager_last[0]               # (losses, gradients) of the last timed step
     mode, ms_step, steps_timed = 'eager', ms_eager, steps
-    try:                                          # the same steps as ONE CUDA graph of R consecutive steps
+    try:                                          # the same steps as CUDA graphs of R consecutive steps
         side = torch.cuda.Stream()
         side.wait_stream(torch.cuda.current_stream())
         with torch.cuda.stream(side):
@@ -673,16 +704,30 @@ def main_config(args, rank, world, local_rank):
                 steps_fn[r]()
         torch.cuda.current_stream().wait_stream(side)
         torch.cuda.synchronize()
-        g = torch.cuda.CUDAGraph()
         keep = []
-        with torch.cuda.graph(g):
-            for r in range(R):
-                keep.append(steps_fn[r]())
+
+        def capture(n):
+            gr = torch.cuda.CUDAGraph()
+            with torch.cuda.graph(gr):
+                for r in range(n):
+                    keep.append(steps_fn[r]())
+            return gr
+        # EXACTLY `steps` steps in the timed region: full graphs of R steps + one tail graph of steps % R
+        full, tail = steps // R, steps % R
+        g = capture(R)
+        g_tail = capture(tail) if tail else None
+
+        def region(_i):
+            for _ in range(full):
+                g.replay()
+            if g_tail is not None:
+                g_tail.replay()
         g.replay()
-        reps = max(steps // R, 1)
-        ms_step = timed(lambda i: g.replay(), reps) / R
-        steps_timed = reps * R
-        mode = f'cuda_graph ({R} steps per graph)'
+        if g_tail is not None:
+            g_tail.replay()
+        ms_step = timed(region, 1) / steps
+        last = keep[-1]
+        mode = f'cuda_graph ({R} steps per graph' + (f' + one tail graph of {tail}' if tail else '') + ')'
     except Exception as e:  # noqa: BLE001
         mode = f'eager (graph capture failed: {type(e).__name__}: {str(e)[:80]})'
     clocks = sampler.stop()
@@ -691,6 +736,11 @@ def main_config(args, rank, world, local_rank):
         if dist is not None:
             dist.destroy_process_group()
         return
+    if args.dump_outputs:
+        losses, grads = last
+        arrays = dict(losses) if isinstance(losses, dict) else {'loss': losses}
+        arrays.update((f'grad_{i}', t) for i, t in enumerate(grads))
+        dump_outputs(args.dump_outputs, arrays)
     peak, peak_src = measured_peak_gbs()
     achieved = info['algo_bytes'] / (ms_step * 1e-3) / 1e9
     imgs = info['images']
@@ -741,16 +791,27 @@ def main_config(args, rank, world, local_rank):
         dist.destroy_process_group()
 
 
+def positive_int(text):
+    v = int(text)
+    if v < 1:
+        raise argparse.ArgumentTypeError(f'{v} is not a positive integer')
+    return v
+
+
 def main():
     ap = argparse.ArgumentParser()
     ap.add_argument('--gpus', type=int, default=1)
-    ap.add_argument('--steps', type=int, default=200)
+    ap.add_argument('--steps', type=positive_int, default=200, help='timed steps')
     ap.add_argument('--warmup', type=int, default=5)
     ap.add_argument('--impl', default='b200', choices=['b200', 'reference'])
     ap.add_argument('--no-cpu-baseline', action='store_true')
     ap.add_argument('--config', default='A', choices=['A', 'C', 'D', 'E'],
                     help='A (default, the headline): BoxInst; C: DiscoBox; D: BoxLevelset; E: Box2Mask (BASELINE.json configs)')
+    ap.add_argument('--dump-outputs', metavar='DIR',
+                    help='after the timed steps, write what the last one returned (losses, gradients) as DIR/<name>.npy')
     args = ap.parse_args()
+    if args.dump_outputs and args.impl == 'reference':
+        ap.error('--dump-outputs writes what the B200 arm computed; --impl reference has no such outputs')
     rank = int(os.environ.get('RANK', 0))
     world = int(os.environ.get('WORLD_SIZE', 1))
     local_rank = int(os.environ.get('LOCAL_RANK', 0))

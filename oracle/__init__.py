@@ -20,9 +20,10 @@ Parity pinning status (see DESIGN.md "Oracle"):
     edge-set fixtures produced from it.
   * The reference's CUDA extensions (``mmdet/ops/pairwise``, ``mmdet/ops/tree_filter``) are compiled
     UNMODIFIED by ``oracle/Makefile`` into ``oracle/_ref/*.so`` (an empty ``THC/THC.h`` shim under
-    ``oracle/csrc/shim`` replaces the header PyTorch no longer ships); they run only on the GPU box:
-    ``tests/test_reference_ext_gpu.py`` compares the product's kernels with them, ``bench.py`` times the
-    reference's GPU loss path around its pairwise op (``gpu_reference``).
+    ``oracle/csrc/shim`` replaces the header PyTorch no longer ships); they run only on a GPU:
+    ``oracle/make_golden_ref_ext.py`` stores their outputs as the golden vectors that
+    ``tests/test_reference_ext_gpu.py`` and ``tests/test_config_a_gpu.py`` compare the product's kernels with,
+    ``bench.py`` times the reference's GPU loss path around its pairwise op (``gpu_reference``).
   * ``skimage.color.rgb2lab`` and ``mmcv.tensor2imgs`` are third-party code absent from
     ``/root/reference`` (scikit-image unpinned; mmcv-full 1.3.17-1.6.0): their published
     algorithms are restated and pinned on known-answer colours + OpenCV's independent

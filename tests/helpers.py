@@ -56,6 +56,38 @@ def rel_err(a, b):
     return ((a - b).norm() / b.norm().clamp(min=1e-30)).item()
 
 
+GOLDEN_FULL = 4096      # a stored reference output with more elements is kept as a seeded sample + projections
+
+
+def projections(t, k=16):
+    """k random projections of the flattened tensor, one per contiguous block of its elements (float64, seeded)."""
+    v = t.detach().double().flatten().cpu()
+    m = -(-v.numel() // k)
+    v = F.pad(v, (0, k * m - v.numel()))
+    r = torch.randn(m, generator=torch.Generator().manual_seed(m), dtype=torch.float64)
+    return (v.view(k, m) @ r).numpy()
+
+
+def check_golden(g, key, t, rtol=None, atol=0.0, rel=None):
+    """``t`` against the reference output stored under ``key`` of the golden file ``g``: allclose(rtol, atol) element-wise on
+    what is stored, and rel_err <= rel on what is stored and, for an output stored as a sample (``key.idx`` / ``key.val``),
+    on the projections of the whole tensor (``key.proj``), so that every element takes part."""
+    t = t.detach().cpu()
+    if key in g:
+        ref, ours = torch.from_numpy(g[key]), t
+        assert ours.shape == ref.shape, (key, ours.shape, ref.shape)
+    else:
+        assert list(t.shape) == g[key + '.shape'].tolist(), (key, t.shape)
+        ref, ours = torch.from_numpy(g[key + '.val']), t.flatten()[torch.from_numpy(g[key + '.idx']).long()]
+    if rtol is not None:
+        assert torch.allclose(ours.to(ref.dtype), ref, rtol=rtol, atol=atol), key
+    if rel is not None:
+        assert rel_err(ours, ref) <= rel, (key, rel_err(ours, ref))
+        if key not in g:
+            err = rel_err(torch.from_numpy(projections(t)), torch.from_numpy(g[key + '.proj']))
+            assert err <= rel, (key, 'projections', err)
+
+
 def host_twin(name):
     """Compiles tests/host_harness/<name>.cpp -- the HOST build of the very header a kernel is made of -- with g++ and
     returns the ctypes handle (test infrastructure: lets the CPU suite check a kernel's arithmetic and indexing bit for bit

@@ -2,22 +2,20 @@
 seed 1234 = the bench inputs): the fused BoxInst mask loss and its gradient against
 
   * the CPU oracle (oracle/boxinst.py: restated CondInstMaskHead.loss, float64), and
-  * the REFERENCE'S OWN compiled CUDA pairwise op (oracle/_ref/pairwise_ext_ref, built by oracle/Makefile from
-    mmdet/ops/pairwise/csrc unmodified) inside a restatement of condinst_head.py:1288-1343 that materialises what the
-    reference materialises.
+  * the REFERENCE'S OWN compiled CUDA pairwise op (mmdet/ops/pairwise/csrc, compiled unmodified by oracle/Makefile) inside
+    a restatement of condinst_head.py:1288-1343 that materialises what the reference materialises, through the golden
+    vectors oracle/make_golden_ref_ext.py stored from it (tests/golden/config_a_reference.npz: both losses, and the
+    gradient as a seeded sample of its elements plus random projections of the whole tensor).
 
 Tolerance: 1e-3 relative on loss and gradient (BASELINE.json north_star); observed ~1e-6."""
-import glob
-import importlib.util
 import os
 
 import pytest
 import torch
 
-from tests.helpers import rel_err
+from tests.helpers import check_golden, rel_err
 
 pytestmark = pytest.mark.gpu
-ROOT = os.path.dirname(os.path.dirname(os.path.abspath(__file__)))
 DEV = 'cuda:0'
 TOL = 1e-3
 
@@ -64,43 +62,9 @@ def test_full_size_against_cpu_oracle(case, ours):
     assert torch.allclose(gx.cpu().double(), g64, rtol=TOL, atol=1e-9)
 
 
-def test_full_size_against_reference_cuda_extension(case, ours):
-    hits = glob.glob(os.path.join(ROOT, 'oracle', '_ref', 'pairwise_ext_ref*.so'))
-    assert hits, 'oracle/_ref/pairwise_ext_ref*.so is missing: run `make -C oracle` where /root/reference exists'
-    spec = importlib.util.spec_from_file_location('pairwise_ext_ref', hits[0])
-    ext = importlib.util.module_from_spec(spec)
-    spec.loader.exec_module(ext)
-    t, (prj, pair, gx) = ours
-    dev = torch.device(DEV)
-
-    class RefPairwise(torch.autograd.Function):            # mmdet/ops/pairwise/pairwise.py:6-26
-        @staticmethod
-        def forward(ctx, logits, size, dilation):
-            pw = ext.pairwise_nlog_forward(size, dilation, logits)
-            ctx.save_for_backward(logits, pw)
-            ctx.cfg = (size, dilation)
-            return pw
-
-        @staticmethod
-        def backward(ctx, g):
-            logits, pw = ctx.saved_tensors
-            return ext.pairwise_nlog_backward(ctx.cfg[0], ctx.cfg[1], logits, pw, g.contiguous()), None, None
-
-    gi = case['gt_inds'].to(dev)
-    sim = t.similarity[case['img_inds'].to(dev)]                       # the G-fold gather of condinst_head.py:1316
-    bm = torch.cat(t.bitmasks())[gi][:, None]
-    x = case['logits'].to(dev).requires_grad_(True)
-
-    def dice(a, b):                                                    # condinst_head.py:117-131
-        a, b = a.flatten(1), b.flatten(1)
-        return 1.0 - 2.0 * (a * b).sum(1) / ((a * a).sum(1) + (b * b).sum(1) + 1e-5)
-
-    scores = x.sigmoid()
-    prj_ref = (dice(scores.max(dim=2, keepdim=True)[0], bm.max(dim=2, keepdim=True)[0]) +
-               dice(scores.max(dim=3, keepdim=True)[0], bm.max(dim=3, keepdim=True)[0])).mean()      # :134-143
-    w = (sim >= 0.3).float() * bm
-    pair_ref = (RefPairwise.apply(x, 3, 2) * w).sum() / w.sum().clamp(min=1.0)                        # :1318-1332
-    (g_ref,) = torch.autograd.grad(prj_ref + pair_ref, x)
-    assert abs(prj.item() - prj_ref.item()) <= TOL * abs(prj_ref.item())
-    assert abs(pair.item() - pair_ref.item()) <= TOL * abs(pair_ref.item())
-    assert rel_err(gx, g_ref) <= TOL
+def test_full_size_against_reference_cuda_extension(golden, ours):
+    ref = golden('config_a_reference')
+    _, (prj, pair, gx) = ours
+    assert abs(prj.item() - ref['loss_prj']) <= TOL * abs(ref['loss_prj'])
+    assert abs(pair.item() - ref['loss_pairwise']) <= TOL * abs(ref['loss_pairwise'])
+    check_golden(ref, 'grad', gx, rel=TOL)
